@@ -34,8 +34,11 @@ def test_every_declared_symbol_is_exported():
 
 
 def test_library_is_sm100a_only():
+    import shutil
     import subprocess
-    out = subprocess.run(["cuobjdump", "-lelf", api.LIB_PATH], capture_output=True, text=True).stdout
+    # the CUDA toolkit's bin directory need not be on PATH (the library's Makefile names nvcc by its full path too)
+    cuobjdump = shutil.which("cuobjdump") or os.path.join(os.environ.get("CUDA_HOME", "/usr/local/cuda"), "bin", "cuobjdump")
+    out = subprocess.run([cuobjdump, "-lelf", api.LIB_PATH], capture_output=True, text=True).stdout
     archs = set(re.findall(r"sm_\d+a?", out))
     assert archs == {"sm_100a"}, archs
 
