@@ -12,7 +12,8 @@
 //                           producer RESOLVES THE SERIAL LOOP'S WALK through its window from every entry position at once
 //                           (pw_resolve, pointer doubling over next(i) = i + (match ? length : 1)): the set of positions the
 //                           loop probes if it arrives at p, and where it leaves the window.  One ring entry per position in
-//                           shared memory: x = {slot, match length, window number}, y = {entry seen, exit}, z = probed set.
+//                           tensor memory: x = {slot, match length}, y = {entry seen, exit}, z = probed set, and one ready
+//                           word per ring slot in shared memory (the window number the slot holds).
 //                           Nothing a producer does depends on the parse except the table entry it happened to read.
 //   walker (1 warp)         the serial loop itself.  Per step it reads the entries of the window it stands in, takes the probed
 //                           set and the exit of its own position, and lets the probed lanes validate and insert themselves:
@@ -23,9 +24,15 @@
 //                           32 bytes and more end a walk and are measured by the walker (pw_extend).  Measured on log text:
 //                           34 bytes per step, 3 % of the steps cut with producers <= 7 windows ahead.
 //
-// The walker never waits for global memory on its common path (ring and table are shared memory), the producers never wait
-// for the walker except for ring space.  Sparse stretches (searchMatchCount > kPwRingSmc: incompressible data) and the last
-// bytes of a block are probed by the walker alone with the batch step of dlz4_parse.cuh while the producers sleep.
+// The walker never waits for global memory on its common path (ring in tensor memory, table in shared memory), the producers
+// never wait for the walker except for ring space.  Sparse stretches (searchMatchCount > kPwRingSmc: incompressible data) and
+// the last bytes of a block are probed by the walker alone with the batch step of dlz4_parse.cuh while the producers sleep.
+//
+// CTA shape: the table of a chain is 32 KiB whatever is done, and seven of them fill the shared memory of an SM; the rings
+// live in tensor memory (TMEM), which nothing else uses.  A warp's tcgen05.ld/st reaches only the TMEM lanes
+// 32 (w % 4) .. +31 of its lane quarter, so the three warps of a team share w % 4: 24 warps, two team slots per quarter,
+// warp w is role (w / 4) % 3 of team (w % 4) + 4 (w / 12).  Slot 7 has no table and no work.  A ring entry's lane is
+// position & 31, the lane of the 32x32b shape.
 //
 // Exactness: a producer's entry is used only under `slot value now == slot value seen`; everything else is decided by the
 // walker from the table it alone writes, in probe order.  Output: the match records of dlz4_parse.cuh (k_encode_blocks
@@ -34,11 +41,14 @@
 
 namespace dlz4 {
 
-constexpr int kPwChains = 6;                  // chains (teams) per CTA: 6 x (32 KiB table + 5.25 KiB ring) of 227 KiB
-constexpr int kPwWin = 14;                    // windows of 32 positions in a chain's ring (what fits beside six tables)
-constexpr int kPwRingBytes = kPwWin * 32 * 12; // a window's entries: three arrays of 32 words (x, y, z below)
-constexpr int kPwCtl = 64;                    // control bytes per chain
-constexpr int kPwChainBytes = kHashEntries * 2 + kPwRingBytes + kPwCtl;
+constexpr int kPwChains = 7;                  // chains (teams) per CTA: 7 x (32 KiB table + 64 B control) of 227 KiB
+constexpr int kPwProducers = 2;               // producer warps per team
+constexpr int kPwThreads = 8 * (1 + kPwProducers) * 32;     // 8 team slots (2 per TMEM lane quarter), the last one idle
+constexpr int kPwWin = 14;                    // windows of 32 positions in a chain's ring
+constexpr uint32_t kPwTmemCols = 128;         // per CTA: 2 teams per lane quarter x 14 windows x 4 columns (x, y, z, unused) = 112
+constexpr int kPwCtl = 64;                    // control bytes per chain (PwCtl)
+constexpr int kPwChainBytes = kHashEntries * 2 + kPwCtl;
+constexpr int kPwSmemBytes = kPwChains * kPwChainBytes + 16;  // + the TMEM address
 constexpr uint32_t kPwRingSmc = 160u;         // the walker uses the ring while searchMatchCount <= this (steps of 1 and 2)
 constexpr uint32_t kPwDone = 0x80000000u, kPwSparse = 0x40000000u;
 constexpr bool kPwPrefetch = true;            // producers prefetch the second stage's lines and the next window pair's source lines
@@ -48,27 +58,55 @@ constexpr bool kPwPrefetch = true;            // producers prefetch the second s
 constexpr uint32_t kPwCap = DLZ4_PW_CAP;              // producers pre-extend a match to this many bytes; the walker continues a longer one
 
 struct PwCtl {                                // one per chain, in shared memory
-    volatile uint32_t w_pos;                  // walker's position (block-relative) | kPwSparse | kPwDone
+    uint32_t w_pos;                           // walker's position (block-relative) | kPwSparse | kPwDone
     volatile uint32_t block;                  // block index of the team, 0xFFFFFFFF: no more work
+    uint32_t ready[kPwWin];                   // ring slot ws holds the entries of window ready[ws] - 1 (0: none yet)
 };
+static_assert(sizeof(PwCtl) <= kPwCtl, "PwCtl");
 
 __device__ __forceinline__ void pw_bar(uint32_t id, uint32_t nthreads) {
     asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(nthreads) : "memory");
 }
-__device__ __forceinline__ uint32_t pw_lds(const uint32_t *p) {
+// The control words order the TMEM accesses of the team's warps: a write is released after tcgen05.wait + fence::before_thread_sync,
+// and a read is acquired before fence::after_thread_sync + the tcgen05 access that depends on it.
+__device__ __forceinline__ uint32_t pw_ld_acquire(const uint32_t *p) {
     uint32_t v;
-    asm volatile("ld.volatile.shared.u32 %0, [%1];" : "=r"(v) : "r"((uint32_t)__cvta_generic_to_shared(p)) : "memory");
+    asm volatile("ld.acquire.cta.shared.u32 %0, [%1];" : "=r"(v) : "r"((uint32_t)__cvta_generic_to_shared(p)) : "memory");
     return v;
 }
-__device__ __forceinline__ void pw_sts(uint32_t *p, const uint32_t v) {
-    asm volatile("st.volatile.shared.u32 [%0], %1;" ::"r"((uint32_t)__cvta_generic_to_shared(p)), "r"(v) : "memory");
+__device__ __forceinline__ void pw_st_release(uint32_t *p, const uint32_t v) {
+    asm volatile("st.release.cta.shared.u32 [%0], %1;" ::"r"((uint32_t)__cvta_generic_to_shared(p)), "r"(v) : "memory");
+}
+__device__ __forceinline__ void pw_st_release2(uint32_t *p, const uint32_t v0, const uint32_t v1) {   // p 8-byte aligned
+    asm volatile("st.release.cta.shared.v2.u32 [%0], {%1, %2};" ::"r"((uint32_t)__cvta_generic_to_shared(p)), "r"(v0), "r"(v1) : "memory");
 }
 __device__ __forceinline__ void pw_prefetch(const void *p) { asm volatile("prefetch.global.L1 [%0];" ::"l"(p)); }
-// ring slot of position p: the words x, y, z of its entry are at slot[0], slot[32], slot[64]
-__device__ __forceinline__ uint32_t pw_slot(const uint32_t p) {
-    const uint32_t w = p >> 5;                                                  // < 2048
-    const uint32_t ws = w - (uint32_t)kPwWin * ((w * 74899u) >> 20);            // w mod 14
-    return ws * 96u + (p & 31u);
+__device__ __forceinline__ void tm_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
+__device__ __forceinline__ void tm_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
+// entries x, y, z of two windows (columns t .. t+7, lane = position & 31): complete when this returns
+__device__ __forceinline__ void tm_st8(const uint32_t t, const uint32_t x0, const uint32_t y0, const uint32_t z0, const uint32_t x1,
+                                       const uint32_t y1, const uint32_t z1) {
+    asm volatile("tcgen05.st.sync.aligned.32x32b.x8.b32 [%0], {%1, %2, %3, %3, %4, %5, %6, %6};\n\t"
+                 "tcgen05.wait::st.sync.aligned;" ::"r"(t), "r"(x0), "r"(y0), "r"(z0), "r"(x1), "r"(y1), "r"(z1) : "memory");
+}
+// loads that complete, and are ordered before what follows, when these return
+__device__ __forceinline__ void tm_ld4(const uint32_t t, uint32_t &x, uint32_t &y, uint32_t &z) {
+    uint32_t u;
+    asm volatile("tcgen05.ld.sync.aligned.32x32b.x4.b32 {%0, %1, %2, %3}, [%4];\n\t"
+                 "tcgen05.wait::ld.sync.aligned;\n\t"
+                 "tcgen05.fence::before_thread_sync;" : "=r"(x), "=r"(y), "=r"(z), "=r"(u) : "r"(t) : "memory");
+}
+__device__ __forceinline__ void tm_ld2(const uint32_t t, uint32_t &x, uint32_t &y) {
+    asm volatile("tcgen05.ld.sync.aligned.32x32b.x2.b32 {%0, %1}, [%2];\n\t"
+                 "tcgen05.wait::ld.sync.aligned;\n\t"
+                 "tcgen05.fence::before_thread_sync;" : "=r"(x), "=r"(y) : "r"(t) : "memory");
+}
+// ring slot of window w (< 2048): w mod 14
+__device__ __forceinline__ uint32_t pw_ws(const uint32_t w) { return w - (uint32_t)kPwWin * ((w * 74899u) >> 20); }
+// Waits (whole warp) until ring slot ws holds window w, then orders the TMEM reads behind.
+__device__ __forceinline__ void pw_wait_ready(const PwCtl *ctl, const uint32_t ws, const uint32_t w, const uint32_t ns) {
+    while (!__all_sync(FULL, pw_ld_acquire(ctl->ready + ws) == w + 1u)) __nanosleep(ns);
+    tm_fence_after();
 }
 // The walk of the serial loop through one aligned window of 32 positions, from every entry position at once (pointer
 // doubling, all lanes): lane i holds the match length ml of position i (0: miss, kPwCap: 64 or more bytes -- the walk ends
@@ -153,7 +191,7 @@ __device__ __forceinline__ uint32_t pw_extend(const uint8_t *__restrict__ base, 
     }
 }
 
-constexpr uint32_t kPwGenMask = 0x7FFu;       // ring entry: x = slot (14 bits) | match length (7) | window number + 1 (11); y = entry seen | exit << 16; z = probed set (pw_resolve)
+// ring entry: x = slot (14 bits) | match length (7) << 14; y = entry seen | exit << 16; z = probed set (pw_resolve)
 
 // candidate bytes (three aligned 16-byte granules, `cs` = byte offset of the first wanted byte inside the first) against
 // the 32 bytes Sw[0..7]: number of equal leading bytes, 0..32.  Branch-free like wide_verify.
@@ -181,7 +219,7 @@ __device__ __forceinline__ uint32_t pw_count32(const uint4 &q0, const uint4 &q1,
 //      independent instruction streams, so the memory round trips (source words, table entry, candidate bytes) overlap.
 //      two == false: window k only (the last window of a block).
 __device__ __forceinline__ void pw_produce2(const uint8_t *__restrict__ base, const uint32_t k, const bool two, const uint16_t *tab,
-                                            uint32_t *ring, const uint32_t lane) {
+                                            const uint32_t tcol, PwCtl *ctl, const uint32_t lane) {
     const uint32_t pa = 32u * k + lane, pb = pa + 32u;
     const uintptr_t ba = reinterpret_cast<uintptr_t>(base);
     const uint32_t a = (uint32_t)(ba & 3u) + pa;
@@ -239,30 +277,27 @@ __device__ __forceinline__ void pw_produce2(const uint8_t *__restrict__ base, co
     }
     uint32_t exa, exb;
     const uint32_t pma = pw_resolve(mla, lane, exa), pmb = pw_resolve(mlb, lane, exb);
-    const uint32_t loa = ha | (mla << 14) | (((k + 1u) & kPwGenMask) << 21);
-    // y and z first, then x with the window number: a reader that sees the number sees the rest
-    uint32_t *const sa = ring + pw_slot(pa), *const sb = ring + pw_slot(pb);
-    pw_sts(sa + 32, seena | (exa << 16));
-    pw_sts(sa + 64, pma);
-    if (two) {
-        pw_sts(sb + 32, seenb | (exb << 16));
-        pw_sts(sb + 64, pmb);
-    }
-    __threadfence_block();
-    pw_sts(sa, loa);
-    if (two) pw_sts(sb, hb | (mlb << 14) | (((k + 2u) & kPwGenMask) << 21));
+    // k is even, so the pair's ring slots ws, ws + 1 are adjacent (kPwWin is even): one store.  The walker has left the
+    // windows these slots held behind (w_pos, read before this call; the fence orders the store after that read).
+    const uint32_t ws = pw_ws(k);
+    __syncwarp();                                                               // (tcgen05.st is warp-collective)
+    tm_fence_after();
+    tm_st8(tcol + 4u * ws, ha | (mla << 14), seena | (exa << 16), pma, hb | (mlb << 14), seenb | (exb << 16), pmb);
+    tm_fence_before();
+    if (two) pw_st_release2(ctl->ready + ws, k + 1u, k + 2u);
+    else pw_st_release(ctl->ready + ws, k + 1u);
 }
 
 // Producer j of kNP takes the window pairs (2j, 2j+1), (2j + 2 kNP, ...), ... -- skipping those the walker has left behind -- and
 // stays at most `lead` windows ahead of the walker's window.
-template <int kNP>
 __device__ __forceinline__ void pw_producer(const uint8_t *__restrict__ base, const uint32_t nwin, const uint32_t lead,
-                                            const uint32_t j, const uint16_t *tab, uint32_t *ring, PwCtl *ctl, const uint32_t lane,
+                                            const uint32_t j, const uint16_t *tab, const uint32_t tcol, PwCtl *ctl, const uint32_t lane,
                                             const uint32_t full_ns) {
+    constexpr int kNP = kPwProducers;
     uint32_t k = 2u * j;
     PT_DECL
     for (;;) {
-        const uint32_t wpos = ctl->w_pos;
+        const uint32_t wpos = pw_ld_acquire(&ctl->w_pos);
         if (wpos & kPwDone) break;
         if (wpos & kPwSparse) { __nanosleep(1024); PT_MARK(8) continue; }
         const uint32_t wk = wpos >> 5;
@@ -271,7 +306,7 @@ __device__ __forceinline__ void pw_producer(const uint8_t *__restrict__ base, co
         if (k >= nwin) { __nanosleep(1024); PT_MARK(8) continue; }
         if (k + 1u >= wk + lead) { __nanosleep(full_ns); PT_MARK(7) continue; }
         if (kPwPrefetch && lane < 2u && k + 2u * (uint32_t)kNP < nwin) pw_prefetch(base + 32u * (k + 2u * (uint32_t)kNP) + 128u * lane);
-        pw_produce2(base, k, k + 1u < nwin, tab, ring, lane);
+        pw_produce2(base, k, k + 1u < nwin, tab, tcol, ctl, lane);
         PT_MARK(6) PT_COUNT(13, 1)
         k += 2u * (uint32_t)kNP;
     }
@@ -280,7 +315,7 @@ __device__ __forceinline__ void pw_producer(const uint8_t *__restrict__ base, co
 
 // ---- walker: the serial loop.  Returns the number of records written.
 __device__ __forceinline__ uint32_t pw_walker(const uint8_t *__restrict__ base, const int32_t len, const uint32_t nwin, uint16_t *tab,
-                                              const uint32_t *ring, PwCtl *ctl, uint64_t *__restrict__ rec, const uint32_t lane) {
+                                              const uint32_t tcol, PwCtl *ctl, uint64_t *__restrict__ rec, const uint32_t lane) {
     const uint32_t lt = (1u << lane) - 1u;
     const int32_t sEnd = len;
     const int32_t mflimit = sEnd - 12;                                          // blockCompress.js:34
@@ -306,21 +341,19 @@ __device__ __forceinline__ uint32_t pw_walker(const uint8_t *__restrict__ base, 
             //      ring entry.  The probed lanes validate (slot unchanged since the producer looked, no two of them in one
             //      slot) and insert themselves; the hits among them are the records.
             const uint32_t s = (uint32_t)sIndex, wbase = s & ~31u, sl = s & 31u;
-            if (pub != wbase) { pub = wbase; if (lane == 0) ctl->w_pos = wbase; }
+            if (pub != wbase) { pub = wbase; if (lane == 0) pw_st_release(&ctl->w_pos, wbase); }
             const uint32_t p = wbase + lane;
-            const uint32_t want = ((p >> 5) + 1u) & kPwGenMask;
-            const uint32_t *slot = ring + pw_slot(p);
-            uint32_t ex;
+            const uint32_t w = wbase >> 5, ws = pw_ws(w);
             PT_MARK(14)
-            for (;;) {
-                ex = pw_lds(slot);
-                if (__all_sync(FULL, (ex >> 21) == want)) break;
+            while (!__all_sync(FULL, pw_ld_acquire(ctl->ready + ws) == w + 1u)) {
                 __nanosleep(32);
                 PT_COUNT(15, 1)
             }
+            tm_fence_after();
+            uint32_t ex, ey, ez;
+            tm_ld4(tcol + 4u * ws, ex, ey, ez);
             PT_MARK(1)
-            const uint32_t ey = pw_lds(slot + 32);
-            const uint32_t PM = pw_lds(slot + 64 + sl - lane), exitp = pw_lds(slot + 32 + sl - lane) >> 16;     // entry of position s
+            const uint32_t PM = __shfl_sync(FULL, ez, sl), exitp = __shfl_sync(FULL, ey, sl) >> 16;     // entry of position s
             const uint32_t seen = ey & 0xFFFFu;
             const uint32_t h = ex & 0x3FFFu, ml = (ex >> 14) & 127u;
             const uint32_t cur = tab[h];                                       // :54 (state before this step)
@@ -398,17 +431,22 @@ __device__ __forceinline__ uint32_t pw_walker(const uint8_t *__restrict__ base, 
             const uint32_t bs = skip_sum(smc);
             const int32_t p = sIndex + (int32_t)(skip_sum(smc + lane) - bs);
             const bool valid = p < rlimit;
-            if (pub != (uint32_t)sIndex) { pub = (uint32_t)sIndex; if (lane == 0) ctl->w_pos = pub; }
-            const uint32_t *slot = ring + pw_slot((uint32_t)p);
-            const uint32_t want = (((uint32_t)p >> 5) + 1u) & kPwGenMask;
-            uint32_t lo;
-            for (;;) {
-                lo = pw_lds(slot);
-                const bool ready = !valid || ((lo >> 21) == want);
-                if (__all_sync(FULL, ready)) break;
-                __nanosleep(20);
+            if (pub != (uint32_t)sIndex) { pub = (uint32_t)sIndex; if (lane == 0) pw_st_release(&ctl->w_pos, pub); }
+            // the valid probes (steps of 1 and 2) lie in at most three windows: each lane takes its entry from the
+            // window's lane p & 31
+            const uint32_t w0 = (uint32_t)sIndex >> 5;
+            const uint32_t wl = (uint32_t)min(__shfl_sync(FULL, p, 31), rlimit - 1) >> 5;
+            uint32_t lo = 0, ye = 0;
+            for (uint32_t w = w0; w <= wl; ++w) {
+                const uint32_t ws = pw_ws(w);
+                pw_wait_ready(ctl, ws, w, 20);
+                uint32_t xw, yw;
+                tm_ld2(tcol + 4u * ws, xw, yw);
+                xw = __shfl_sync(FULL, xw, (uint32_t)p & 31u);
+                yw = __shfl_sync(FULL, yw, (uint32_t)p & 31u);
+                if (((uint32_t)p >> 5) == w) { lo = xw; ye = yw; }
             }
-            const uint32_t seen = pw_lds(slot + 32) & 0xFFFFu;
+            const uint32_t seen = ye & 0xFFFFu;
             const uint32_t h = lo & 0x3FFFu, ml = (lo >> 14) & 127u;
             const uint32_t cur = tab[h];                                       // :54 (state before this step)
             const uint32_t claim = __ballot_sync(FULL, valid && ml != 0u);
@@ -479,7 +517,7 @@ __device__ __forceinline__ uint32_t pw_walker(const uint8_t *__restrict__ base, 
         // ---- batch step (sparse schedule, block tail): the walker alone, from global memory; producers sleep
         if (smc > kPwRingSmc && sIndex < rlimit) {
             const uint32_t v = (uint32_t)sIndex | kPwSparse;
-            if (pub != v) { pub = v; if (lane == 0) ctl->w_pos = pub; }
+            if (pub != v) { pub = v; if (lane == 0) pw_st_release(&ctl->w_pos, pub); }
         }
         const uint32_t base_sum = skip_sum(smc);
         const int32_t p = sIndex + (int32_t)(skip_sum(smc + lane) - base_sum);
@@ -528,67 +566,89 @@ __device__ __forceinline__ uint32_t pw_walker(const uint8_t *__restrict__ base, 
     return nrec;
 }
 
-// Fresh independent blocks <= 64 KiB as producer/walker teams.  CTA = kPwChains teams; warp t of a team: 0 = walker,
-// 1..kNP = producers.  Output: the match records of every block and their number, for k_encode_blocks.  (An encoder warp
-// inside the team was measured: it delays the team's next block; the encoder stays a kernel of its own.)
-template <int kNP>
-__global__ void __launch_bounds__(kPwChains * (1 + kNP) * 32, 1)
+// Fresh independent blocks <= 64 KiB as producer/walker teams.  CTA = kPwChains teams (warp -> team: header); role 0 of a
+// team = walker, 1..kPwProducers = producers.  Output: the match records of every block and their number, for
+// k_encode_blocks.  (An encoder warp inside the team was measured: it delays the team's next block; the encoder stays a
+// kernel of its own.)
+__global__ void __launch_bounds__(kPwThreads, 1)
 k_parse_pw(const uint8_t *__restrict__ src, const uint64_t *__restrict__ src_off, const uint32_t *__restrict__ src_len,
            uint32_t nblocks, uint64_t *__restrict__ rec_base, uint64_t rec_stride /* records per block */,
            uint32_t *__restrict__ nrec_out, uint32_t *counter, uint32_t lead,
            uint32_t full_ns /* a producer with a full ring sleeps this long: the ring buffers several windows */) {
     extern __shared__ __align__(16) uint8_t smem[];
-    constexpr uint32_t kRoles = 1 + kNP;
+    constexpr uint32_t kRoles = 1 + kPwProducers;
     constexpr uint32_t kTeam = kRoles * 32;
     const uint32_t lane = lane_id(), warp = threadIdx.x >> 5;
-    const uint32_t chain = warp / kRoles, role = warp % kRoles;
-    const uint32_t tid = threadIdx.x - chain * kTeam;                          // thread index inside the team
-    uint8_t *const cb = smem + (size_t)chain * kPwChainBytes;
-    uint16_t *const tab = reinterpret_cast<uint16_t *>(cb);
-    uint32_t *const ring = reinterpret_cast<uint32_t *>(cb + kHashEntries * 2);
-    PwCtl *const ctl = reinterpret_cast<PwCtl *>(cb + kHashEntries * 2 + kPwRingBytes);
-    const uint32_t bar = 1u + chain;
-    // first block of a team: spread over the CTAs first, then over the teams of a CTA; later ones from the queue
-    uint32_t first = chain * gridDim.x + blockIdx.x;
-    const uint32_t qbase = gridDim.x * (uint32_t)kPwChains;
-    bool have_first = true;
-    for (;;) {
-        pw_bar(bar, kTeam);                                                    // everyone is done with the previous block
-        if (role == 0 && lane == 0) {
-            uint32_t b;
-            if (have_first) b = first; else b = qbase + atomicAdd(counter, 1u);
-            ctl->block = b < nblocks ? b : 0xFFFFFFFFu;
-            ctl->w_pos = 0u;
-        }
-        have_first = false;
-        pw_bar(bar, kTeam);
-        const uint32_t b = ctl->block;
-        if (b == 0xFFFFFFFFu) return;
-        const uint32_t len = src_len[b];
-        if (len > 65536u) {
-            if (role == 0 && lane == 0) nrec_out[b] = 0xFFFFFFFFu;
-            continue;
-        }
-        {   // empty table (bufferCompress.js:182 / :235), invalid ring
-            uint4 *z = reinterpret_cast<uint4 *>(cb);
-            for (uint32_t i = tid; i < (kHashEntries * 2 + kPwRingBytes) / 16; i += kTeam) z[i] = make_uint4(0, 0, 0, 0);
-        }
-        pw_bar(bar, kTeam);
-        const uint8_t *base = src + src_off[b];
-        uint64_t *const rec = rec_base + (uint64_t)b * rec_stride;
-        // windows whose loads stay inside the block: position 32k+31 reads its own bytes up to +71 and, for a candidate right
-        // below it, 16-byte granules up to +79
-        const uint32_t nwin = len >= 112u ? (len - 111u) / 32u + 1u : 0u;
-        if (role == 0) {
-            const uint32_t n = pw_walker(base, (int32_t)len, nwin, tab, ring, ctl, rec, lane);
-            if (lane == 0) {
-                nrec_out[b] = n;
-                ctl->w_pos = kPwDone;
+    const uint32_t quarter = warp & 3u, tslot = (warp >> 2) / kRoles, role = (warp >> 2) % kRoles;
+    const uint32_t chain = quarter + 4u * tslot;
+    uint32_t *const taddr_smem = reinterpret_cast<uint32_t *>(smem + kPwChains * kPwChainBytes);
+    if (warp == 0) {
+        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;\n\t"
+                     "tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;"
+                     ::"r"((uint32_t)__cvta_generic_to_shared(taddr_smem)), "r"(kPwTmemCols) : "memory");
+    }
+    tm_fence_before();
+    __syncthreads();
+    tm_fence_after();
+    const uint32_t taddr = *taddr_smem;
+    // column 0 of the team's ring in its lane quarter
+    const uint32_t tcol = taddr + ((32u * quarter) << 16) + tslot * (uint32_t)(kPwWin * 4);
+    if (chain < (uint32_t)kPwChains) {
+        const uint32_t tid = role * 32u + lane;                                 // thread index inside the team
+        uint8_t *const cb = smem + (size_t)chain * kPwChainBytes;
+        uint16_t *const tab = reinterpret_cast<uint16_t *>(cb);
+        PwCtl *const ctl = reinterpret_cast<PwCtl *>(cb + kHashEntries * 2);
+        const uint32_t bar = 1u + chain;
+        // first block of a team: spread over the CTAs first, then over the teams of a CTA; later ones from the queue
+        uint32_t first = chain * gridDim.x + blockIdx.x;
+        const uint32_t qbase = gridDim.x * (uint32_t)kPwChains;
+        bool have_first = true;
+        for (;;) {
+            pw_bar(bar, kTeam);                                                // everyone is done with the previous block
+            if (role == 0 && lane == 0) {
+                uint32_t b;
+                if (have_first) b = first; else b = qbase + atomicAdd(counter, 1u);
+                ctl->block = b < nblocks ? b : 0xFFFFFFFFu;
+                ctl->w_pos = 0u;
             }
-        } else {
-            pw_producer<kNP>(base, nwin, lead, role - 1u, tab, ring, ctl, lane, full_ns);
+            have_first = false;
+            pw_bar(bar, kTeam);
+            const uint32_t b = ctl->block;
+            if (b == 0xFFFFFFFFu) break;
+            const uint32_t len = src_len[b];
+            if (len > 65536u) {
+                if (role == 0 && lane == 0) nrec_out[b] = 0xFFFFFFFFu;
+                continue;
+            }
+            {   // empty table (bufferCompress.js:182 / :235), empty ring (the ready words gate every TMEM read)
+                uint4 *z = reinterpret_cast<uint4 *>(cb);
+                for (uint32_t i = tid; i < kHashEntries * 2 / 16; i += kTeam) z[i] = make_uint4(0, 0, 0, 0);
+                if (tid < (uint32_t)kPwWin) ctl->ready[tid] = 0u;
+            }
+            pw_bar(bar, kTeam);
+            const uint8_t *base = src + src_off[b];
+            uint64_t *const rec = rec_base + (uint64_t)b * rec_stride;
+            // windows whose loads stay inside the block: position 32k+31 reads its own bytes up to +71 and, for a candidate
+            // right below it, 16-byte granules up to +79
+            const uint32_t nwin = len >= 112u ? (len - 111u) / 32u + 1u : 0u;
+            if (role == 0) {
+                const uint32_t n = pw_walker(base, (int32_t)len, nwin, tab, tcol, ctl, rec, lane);
+                if (lane == 0) {
+                    nrec_out[b] = n;
+                    pw_st_release(&ctl->w_pos, kPwDone);
+                }
+            } else {
+                pw_producer(base, nwin, lead, role - 1u, tab, tcol, ctl, lane, full_ns);
+            }
         }
     }
+    // every warp, the idle slot's too: the TMEM is freed when no team uses it any more (a CTA that exits without the
+    // dealloc leaves its columns taken for the next kernel on the SM)
+    tm_fence_before();
+    __syncthreads();
+    tm_fence_after();
+    if (warp == 0)
+        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(kPwTmemCols) : "memory");
 }
 
 }  // namespace dlz4
