@@ -1497,7 +1497,7 @@ k_decompress_blocks(const uint8_t *__restrict__ src, const uint64_t *__restrict_
 __global__ void __launch_bounds__(32)
 k_decompress_chain(const uint8_t *__restrict__ src, const uint64_t *__restrict__ src_off,
                    const uint32_t *__restrict__ src_len, const uint8_t *__restrict__ stored, uint32_t nblocks,
-                   uint8_t *dst, uint64_t dst_total, const uint8_t *__restrict__ dict, uint32_t dict_len,
+                   uint8_t *dst, uint64_t dst_total, uint32_t block_max, const uint8_t *__restrict__ dict, uint32_t dict_len,
                    uint32_t *__restrict__ out_len, uint8_t *__restrict__ status, uint64_t *total_out) {
     const uint32_t lane = lane_id();
     int64_t op = 0;
@@ -1505,14 +1505,15 @@ k_decompress_chain(const uint8_t *__restrict__ src, const uint64_t *__restrict__
     for (uint32_t b = 0; b < nblocks; ++b) {
         uint32_t w = 0;
         if (st == ST_OK) {
+            // a block never decodes past blockMaxSize, like the jump decoder's (LZ4 frame format; liblz4 enforces it too)
+            const uint64_t left = dst_total - (uint64_t)op, room = left < block_max ? left : block_max;
             if (stored[b]) {
                 w = src_len[b];
-                if (op + w > (int64_t)dst_total) { st = ST_OUTPUT_TOO_SMALL; w = 0; }
+                if (w > room) { st = ST_OUTPUT_TOO_SMALL; w = 0; }
                 else warp_copy(dst + op, src + src_off[b], w, lane);
                 __syncwarp();
             } else {
-                const uint64_t room = dst_total - (uint64_t)op;
-                w = decompress_block_warp_v2<true>(src + src_off[b], src_len[b], dst + op, (uint32_t)(room < 0xFFFFFFFFull ? room : 0xFFFFFFFFull),
+                w = decompress_block_warp_v2<true>(src + src_off[b], src_len[b], dst + op, (uint32_t)room,
                                              (uint32_t)(op < 65536 ? op : 65536), dict, dict_len, &st);
             }
         }
@@ -2017,6 +2018,61 @@ k_jd_bases(const uint32_t *__restrict__ out_len, const uint32_t *__restrict__ re
         acc += out_len[b];
     }
     base[nblocks] = acc;
+}
+
+// Error path of the jump decoder: the first block with any problem (the host finds it in k_jd_bases's statuses) gets the
+// status the reference's token loop reaches first -- dec_one_sequence without the copies.  The scans and k_jd_bases test
+// capacity, lengths, offsets and history at different times, so they may name a later error of that block (or another
+// block's).  A status depends only on lengths, offsets and positions, never on decoded bytes.  hist = how far before the
+// block's output its history reaches (dictionary, plus the earlier output when linked); room = the block's capacity.
+// Blocks before this one are clean: scan OK, reach within their history, output within the capacity.
+__global__ void __launch_bounds__(32)
+k_jd_status(const uint8_t *__restrict__ src, const uint64_t *__restrict__ src_off, const uint32_t *__restrict__ src_len,
+            const uint8_t *__restrict__ stored, uint64_t hist, uint64_t room, uint8_t *status) {
+    if (threadIdx.x) return;
+    const uint8_t *in = src + *src_off;
+    const uint32_t n = *src_len;
+    uint32_t st = ST_OK;
+    if (*stored) {
+        if (n > room) st = ST_OUTPUT_TOO_SMALL;
+    } else {
+        uint32_t ip = 0;
+        uint64_t op = 0;
+        while (ip < n) {
+            const uint32_t token = in[ip++];                     // :58
+            uint64_t lit = token >> 4;
+            if (lit == 15u) {                                    // :62-68
+                uint32_t v;
+                do {
+                    if (ip >= n) { st = ST_MALFORMED; goto done; }
+                    v = in[ip++]; lit += v;
+                } while (v == 255u);
+            }
+            if (op + lit > room) { st = ST_OUTPUT_TOO_SMALL; break; }                     // :74
+            if ((uint64_t)ip + lit > n) { st = ST_MALFORMED; break; }                    // :75
+            ip += (uint32_t)lit;
+            op += lit;
+            if (ip >= n) break;                                  // :123
+            if (ip + 2 > n) { st = ST_MALFORMED; break; }
+            const uint32_t offset = (uint32_t)in[ip] | ((uint32_t)in[ip + 1] << 8);      // :126
+            ip += 2;
+            if (offset == 0) { st = ST_OFFSET_ZERO; break; }    // :128
+            uint64_t ml = token & 15u;
+            if (ml == 15u) {                                     // :132-138
+                uint32_t v;
+                do {
+                    if (ip >= n) { st = ST_MALFORMED; goto done; }
+                    v = in[ip++]; ml += v;
+                } while (v == 255u);
+            }
+            ml += 4;
+            if (op + hist < offset) { st = ST_DICT_OOB; break; }                        // :150-152, before the match capacity
+            if (op + ml > room) { st = ST_OUTPUT_TOO_SMALL; break; }
+            op += ml;
+        }
+    }
+done:
+    if (st != ST_OK) *status = (uint8_t)st;                      // (the walk finds an error whenever k_jd_bases did)
 }
 
 // One unit = blocks [b0, b1).  P is indexed from the unit's first output byte.

@@ -48,7 +48,8 @@ extern "C" {
 #define DLZ4_HIST_RAW      0   /* every block has its own output base; history = dictionary only
                                   (decompressBlock(msg,0,len,out_i,0,dict), blockDecompress.js:142-147) */
 #define DLZ4_HIST_FRAME    1   /* all blocks write one output buffer; block history = dictionary ++ dst[0..dst_off[i])
-                                  (bufferDecompress.js:153) */
+                                  (bufferDecompress.js:153), the caller's bytes of dst included: the host-pointer variant
+                                  uploads all of dst in this mode */
 
 typedef struct dlz4_ctx dlz4_ctx;
 

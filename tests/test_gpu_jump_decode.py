@@ -78,15 +78,11 @@ def test_corrupt_linked_frames_raise_the_reference_errors(dl):
     pos = len(g) // 2
     for k in range(pos, pos + 4000):
         g[k] = 0
-    for frame in (g,):
-        try:
-            want = oracle.decompress_buffer(bytes(frame))
-            got = dl.decompressBuffer(bytes(frame))
-            assert got == want
-        except oracle.OracleError as e:
-            with pytest.raises(dl.LZ4Error) as ei:
-                dl.decompressBuffer(bytes(frame))
-            assert str(e).split(":")[-1].strip().lower() in str(ei.value).lower() or True
+    with pytest.raises(oracle.OracleError) as want:
+        oracle.decompress_buffer(bytes(g))
+    with pytest.raises(dl.LZ4Error) as ei:
+        dl.decompressBuffer(bytes(g))
+    assert ei.value.status == -want.value.code and str(ei.value) == str(want.value)
     # truncated frame
     with pytest.raises(dl.LZ4Error):
         dl.decompressBuffer(bytes(f[: len(f) // 3]))
