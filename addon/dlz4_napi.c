@@ -13,6 +13,11 @@
  *   xxHash32(input, seed) -> u32                                                            xxhash32.js:21
  *   frameCompressAsync / frameDecompressAsync(...) -> Promise                               workerClient.js:114-152 (LZ4Worker)
  *   allocPinned(bytes) -> Uint8Array over page-locked memory                                (outputBuffer at the full PCIe rate)
+ *   compressBatch(src, srcOff, srcLen, dict, maxBlockSize, blockIndependence, contentChecksum, addContentSize, output,
+ *                 blockChecksum, frameOff) -> total bytes        frameCompress once per message, one GPU pass (many messages)
+ *   decompressBatch(src, frameOff, frameLen, dict, flags, output, dstOff, dstCap, outLen, status) -> first non-zero status
+ *                                                              frameDecompress once per frame; per-frame statuses in `status`
+ *   (offsets / lengths / capacities of the batch calls are BigUint64Array, srcLen a Uint32Array, status a Uint8Array)
  */
 #ifdef DLZ4_NAPI_SYNTAX_ONLY
 #include "node_api_stub.h"
@@ -156,6 +161,64 @@ static napi_value FrameDecompress(napi_env env, napi_callback_info info) {
     if (st) return fail(env, st, (int)fi.version);
     napi_create_typedarray(env, napi_uint8_array, (size_t)n, ab, 0, &view);      /* result.subarray(0, n), bufferDecompress.js:219 */
     return view;
+}
+
+/* typed array of type `want` with at least `count` elements -> pointer */
+static int typed(napi_env env, napi_value v, napi_typedarray_type want, size_t count, void **p) {
+    napi_typedarray_type t;
+    napi_value ab;
+    size_t n = 0, off = 0;
+    bool is_ta = false;
+    if (napi_is_typedarray(env, v, &is_ta) != napi_ok || !is_ta) return 0;
+    if (napi_get_typedarray_info(env, v, &t, &n, p, &ab, &off) != napi_ok) return 0;
+    return t == want && n >= count;
+}
+
+/* frameCompress over many messages (dlz4_frames_compress_batch): message i = src[srcOff[i] .. +srcLen[i]); its frame is
+ * output[frameOff[i] .. frameOff[i+1]) (frameOff has n + 1 entries; output needs the sum of the messages' frame bounds). */
+static napi_value CompressBatch(napi_env env, napi_callback_info info) {
+    ARGS(11);
+    uint8_t *src, *dict = NULL, *out;
+    size_t nsrc, nd = 0, nout, n = 0;
+    void *off, *len, *foff;
+    napi_typedarray_type t;
+    napi_value ab;
+    size_t boff;
+    dlz4_frame_opts o;
+    if (argc < 11 || !u8(env, a[0], &src, &nsrc) || !u8(env, a[3], &dict, &nd) || !u8(env, a[8], &out, &nout)) return BAD_ARG();
+    if (napi_get_typedarray_info(env, a[2], &t, &n, &len, &ab, &boff) != napi_ok || t != napi_uint32_array) return BAD_ARG();
+    if (!typed(env, a[1], napi_biguint64_array, n, &off) || !typed(env, a[10], napi_biguint64_array, n + 1, &foff)) return BAD_ARG();
+    frame_opts(env, a + 2, argc - 2, &o);
+    int st = dlz4_frames_compress_batch(g_ctx, src, nsrc, (const uint64_t *)off, (const uint32_t *)len, (uint32_t)n, dict, (uint32_t)nd, &o,
+                                        out, nout, (uint64_t *)foff);
+    if (st) return fail(env, st, 0);
+    napi_value r;
+    napi_create_double(env, (double)((uint64_t *)foff)[n], &r);
+    return r;
+}
+
+/* frameDecompress over many frames (dlz4_frames_decompress_batch): frame i = src[frameOff[i] .. +frameLen[i]) decodes to
+ * output[dstOff[i] .. +dstCap[i]); outLen[i] / status[i] as frameDecompress would end (status 0 or a DLZ4_E_* code; the JS
+ * side throws per frame).  Throws only for an invalid call or a CUDA failure. */
+static napi_value DecompressBatch(napi_env env, napi_callback_info info) {
+    ARGS(10);
+    uint8_t *src, *dict = NULL, *out, *status;
+    size_t nsrc, nd = 0, nout, n = 0, nst = 0;
+    void *foff, *flen, *doff, *dcap, *olen;
+    uint32_t flags = 1;
+    if (argc < 10 || !u8(env, a[0], &src, &nsrc) || !u8(env, a[3], &dict, &nd) || !u8(env, a[5], &out, &nout) ||
+        !u8(env, a[9], &status, &nst)) return BAD_ARG();
+    n = nst;
+    napi_get_value_uint32(env, a[4], &flags);
+    if (!typed(env, a[1], napi_biguint64_array, n, &foff) || !typed(env, a[2], napi_biguint64_array, n, &flen) ||
+        !typed(env, a[6], napi_biguint64_array, n, &doff) || !typed(env, a[7], napi_biguint64_array, n, &dcap) ||
+        !typed(env, a[8], napi_biguint64_array, n, &olen)) return BAD_ARG();
+    int st = dlz4_frames_decompress_batch(g_ctx, src, nsrc, (const uint64_t *)foff, (const uint64_t *)flen, (uint32_t)n, dict, (uint32_t)nd,
+                                          flags, out, nout, (const uint64_t *)doff, (const uint64_t *)dcap, (uint64_t *)olen, status);
+    if (st >= DLZ4_E_INVALID_ARG) return fail(env, st, 0);
+    napi_value r;
+    napi_create_double(env, (double)st, &r);
+    return r;
 }
 
 static napi_value XxHash32(napi_env env, napi_callback_info info) {
@@ -303,6 +366,8 @@ NAPI_MODULE_INIT() {
         {"frameCompressAsync", 0, FrameCompressAsync, 0, 0, 0, napi_default, 0},
         {"frameDecompressAsync", 0, FrameDecompressAsync, 0, 0, 0, napi_default, 0},
         {"allocPinned", 0, AllocPinned, 0, 0, 0, napi_default, 0},
+        {"compressBatch", 0, CompressBatch, 0, 0, 0, napi_default, 0},
+        {"decompressBatch", 0, DecompressBatch, 0, 0, 0, napi_default, 0},
     };
     napi_define_properties(env, exports, sizeof d / sizeof d[0], d);
     return exports;

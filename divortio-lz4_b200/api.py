@@ -25,7 +25,8 @@ __all__ = [
     "LZ4", "LZ4Error", "Context", "default_context", "compressBlock", "decompressBlock", "compressBuffer",
     "decompressBuffer", "xxHash32", "compress_blocks", "decompress_blocks", "xxh32_batch", "compress_bound",
     "frame_bound", "shard_range", "ensureBuffer", "lib", "LIB_PATH", "WARM_NONE", "WARM_JENKINS", "WARM_TABLE",
-    "HIST_RAW", "HIST_FRAME", "frame_info", "decompressFrames", "XXHash32", "chain_compress",
+    "HIST_RAW", "HIST_FRAME", "frame_info", "decompressFrames", "XXHash32", "chain_compress", "compressBuffers",
+    "decompressBuffers",
 ]
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
@@ -123,6 +124,12 @@ def lib():
         "dlz4_frame_header": (C.c_size_t, [C.POINTER(FrameOpts), u64, C.c_int, u32, vp]),
         "dlz4_frame_decompress_range": (C.c_int, [vp, vp, u64, u32, u32, vp, u64, u32, vp, u64, C.POINTER(u64), vp]),
         "dlz4_xxh32_update_resident": (C.c_int, [vp, C.POINTER(Xxh32State), C.c_int]),
+        "dlz4_frames_compress_batch_dev": (C.c_int, [vp, vp, vp, vp, u32, u32, vp, u32, C.POINTER(FrameOpts), vp, u64, vp, vp]),
+        "dlz4_frames_compress_batch": (C.c_int, [vp, vp, u64, vp, vp, u32, vp, u32, C.POINTER(FrameOpts), vp, u64, vp]),
+        "dlz4_frames_batch_info_dev": (C.c_int, [vp, vp, vp, vp, u32, vp, vp, vp]),
+        "dlz4_frames_batch_info": (C.c_int, [vp, vp, u64, vp, vp, u32, vp, vp]),
+        "dlz4_frames_decompress_batch_dev": (C.c_int, [vp, vp, vp, vp, u32, vp, u32, u32, vp, vp, vp, vp, vp, vp]),
+        "dlz4_frames_decompress_batch": (C.c_int, [vp, vp, u64, vp, vp, u32, vp, u32, u32, vp, u64, vp, vp, vp, vp]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(L, name)
@@ -139,7 +146,8 @@ EXPORTED_SYMBOLS = [
     "dlz4_compress_block", "dlz4_decompress_block", "dlz4_xxh32_batch_dev", "dlz4_xxh32_stream_dev", "dlz4_xxh32", "dlz4_xxh32_async", "dlz4_xxh32_wait",
     "dlz4_xxh32_batch", "dlz4_frame_compress", "dlz4_frame_info", "dlz4_frame_decompress", "dlz4_frame_pack_dev", "dlz4_frames_decompress", "dlz4_frames_info", "dlz4_frame_decompress_ex", "dlz4_xxh32_reset", "dlz4_xxh32_update", "dlz4_xxh32_digest",
     "dlz4_chain_compress", "dlz4_stream_blocks", "dlz4_frame_body_compress", "dlz4_frame_body_fetch", "dlz4_frame_header", "dlz4_frame_decompress_range",
-    "dlz4_xxh32_update_resident",
+    "dlz4_xxh32_update_resident", "dlz4_frames_compress_batch_dev", "dlz4_frames_compress_batch", "dlz4_frames_batch_info_dev",
+    "dlz4_frames_batch_info", "dlz4_frames_decompress_batch_dev", "dlz4_frames_decompress_batch",
 ]
 
 
@@ -437,6 +445,102 @@ def decompressFrames(input, dictionary=None, verifyChecksum=True, verifyBlockChe
                                       _ptr(out), int(total.value), C.byref(n), C.byref(count))
     ctx.check(st)
     return out[:int(n.value)].tobytes(), int(count.value)
+
+
+def frame_opts(maxBlockSize=4194304, blockIndependence=False, contentChecksum=False, addContentSize=True, blockChecksum=False):
+    """The dlz4_frame_opts of compressBuffer's arguments."""
+    return FrameOpts(int(maxBlockSize or 0) & 0xFFFFFFFF if (maxBlockSize or 0) < 2 ** 32 else 0xFFFFFFFF,
+                     int(bool(blockIndependence)), int(bool(contentChecksum)), int(bool(addContentSize)), int(bool(blockChecksum)))
+
+
+def _concat(items):
+    """Packs a list of byte-likes into one uint8 array: (array, offsets u64, lengths)."""
+    arrs = [ensureBuffer(x) for x in items]
+    lens = np.array([a.size for a in arrs], dtype=np.uint64)
+    off = np.zeros(len(arrs), dtype=np.uint64)
+    if len(arrs) > 1:
+        off[1:] = np.cumsum(lens)[:-1]
+    buf = np.concatenate(arrs) if arrs else np.zeros(0, dtype=np.uint8)
+    return np.ascontiguousarray(buf, dtype=np.uint8), off, lens
+
+
+def _frame_error(status, frame):
+    """LZ4Error of a frame's status, with the version read from its FLG byte for "Unsupported Version N"."""
+    extra = ""
+    if status == E_BAD_VERSION:
+        f = ensureBuffer(frame)
+        extra = " %d" % ((int(f[4]) & 0xC0) >> 6 if f.size >= 5 else 0)
+    return LZ4Error(status, lib().dlz4_strerror(status).decode() + extra)
+
+
+def compressBuffers(inputs, dictionary=None, maxBlockSize=4194304, blockIndependence=False, contentChecksum=False,
+                    addContentSize=True, blockChecksum=False, ctx=None):
+    """compressBuffer over many inputs in one GPU pass (dlz4_frames_compress_batch): one frame per input, each byte-identical
+    to compressBuffer(input, dictionary, ...) with the same options.  Returns a list of bytes."""
+    ctx = ctx or default_context()
+    src, off, lens = _concat(inputs)
+    n = len(lens)
+    if n == 0:
+        return []
+    d = ensureBuffer(dictionary) if dictionary is not None and len(dictionary) > 0 else None
+    opts = frame_opts(maxBlockSize, blockIndependence, contentChecksum, addContentSize, blockChecksum)
+    lens32 = lens.astype(np.uint32)
+    if (lens >= 0x7FFF0000).any():
+        ctx.check(21)
+    cap = int((19 + lens + (lens // 65536 + 1) * 8 + 8 + 64).sum())
+    dst = np.empty(cap, dtype=np.uint8)
+    frame_off = np.zeros(n + 1, dtype=np.uint64)
+    st = lib().dlz4_frames_compress_batch(ctx.handle, _ptr(src), src.size, _ptr(off), _ptr(lens32), n, _ptr(d),
+                                          d.size if d is not None else 0, C.byref(opts), _ptr(dst), cap, _ptr(frame_off))
+    ctx.check(st)
+    fo = frame_off.tolist()
+    mv = dst.tobytes()
+    return [mv[fo[i]:fo[i + 1]] for i in range(n)]
+
+
+def decompressBuffers(frames, dictionary=None, verifyChecksum=True, verifyBlockChecksums=False, errors="raise", ctx=None):
+    """decompressBuffer over many frames in one GPU pass (dlz4_frames_batch_info + dlz4_frames_decompress_batch).  Entry i is
+    what decompressBuffer(frames[i], ...) returns.  errors="raise": the first failing frame's LZ4Error is raised;
+    errors="return": a failing frame's entry is its LZ4Error."""
+    if errors not in ("raise", "return"):
+        raise ValueError('errors must be "raise" or "return"')
+    ctx = ctx or default_context()
+    src, off, lens = _concat(frames)
+    n = len(lens)
+    if n == 0:
+        return []
+    L = lib()
+    max_dec = np.zeros(n, dtype=np.uint64)
+    info_st = np.zeros(n, dtype=np.uint8)
+    ctx.check(L.dlz4_frames_batch_info(ctx.handle, _ptr(src), src.size, _ptr(off), _ptr(lens), n, _ptr(max_dec), _ptr(info_st)))
+    dst_cap = max_dec
+    dst_off = np.zeros(n, dtype=np.uint64)
+    if n > 1:
+        dst_off[1:] = np.cumsum(dst_cap)[:-1]
+    total = int(dst_cap.sum())
+    dst = np.empty(total + 16, dtype=np.uint8)
+    out_len = np.zeros(n, dtype=np.uint64)
+    status = np.zeros(n, dtype=np.uint8)
+    d = ensureBuffer(dictionary) if dictionary is not None and len(dictionary) > 0 else None
+    flags = (1 if verifyChecksum else 0) | (2 if verifyBlockChecksums else 0)
+    st = L.dlz4_frames_decompress_batch(ctx.handle, _ptr(src), src.size, _ptr(off), _ptr(lens), n, _ptr(d),
+                                        d.size if d is not None else 0, flags, _ptr(dst), dst.size, _ptr(dst_off), _ptr(dst_cap),
+                                        _ptr(out_len), _ptr(status))
+    if st == E_CUDA or st >= 20:
+        ctx.check(st)
+    out = []
+    mv = dst.tobytes()
+    for i in range(n):
+        s = int(info_st[i]) or int(status[i])               # decompressBuffer raises frame_info's error first
+        if s:
+            e = _frame_error(s, frames[i])
+            if errors == "raise":
+                raise e
+            out.append(e)
+        else:
+            o = int(dst_off[i])
+            out.append(mv[o:o + int(out_len[i])])
+    return out
 
 
 class XXHash32(object):

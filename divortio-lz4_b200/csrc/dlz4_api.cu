@@ -3,6 +3,7 @@
 // compressed, decoded and hashed on the GPU.  There is no CPU path.
 #include "../../include/dlz4_b200.h"
 #include "dlz4_kernels.cuh"
+#include "dlz4_frames.cuh"
 
 #include <algorithm>
 #include <atomic>
@@ -40,5 +41,6 @@ extern "C" {
 #include "api_xxh32.inc"
 #include "api_frame_compress.inc"
 #include "api_frame_decompress.inc"
+#include "api_frame_batch.inc"
 #include "api_stream.inc"
 }  // extern "C"

@@ -60,3 +60,25 @@ def xxh32_stream_dev(ctx, data, out, seed=0):
 def frame_pack_dev(ctx, src, src_off, src_len, comp, comp_off, comp_len, block_checksum, segment, block_pos):
     ctx.check(api.lib().dlz4_frame_pack_dev(ctx.handle, _p(src), _p(src_off), _p(src_len), _p(comp), _p(comp_off), _p(comp_len),
                                             src_off.numel(), int(block_checksum), _p(segment), _p(block_pos), _stream()))
+
+
+def frames_compress_batch_dev(ctx, src, src_off, src_len, max_len, dst, frame_off, opts, dictionary=None):
+    """dlz4_frames_compress_batch_dev on the current torch stream.  src/dst/dictionary uint8, src_off int64, src_len int32,
+    frame_off int64[nframes + 1] (CUDA tensors); opts an api.FrameOpts (api.frame_opts(...))."""
+    ctx.check(api.lib().dlz4_frames_compress_batch_dev(ctx.handle, _p(src), _p(src_off), _p(src_len), src_off.numel(), int(max_len),
+                                                       _p(dictionary), dictionary.numel() if dictionary is not None else 0,
+                                                       C.byref(opts), _p(dst), dst.numel(), _p(frame_off), _stream()))
+
+
+def frames_batch_info_dev(ctx, src, frame_off, frame_len, max_decoded, status):
+    """dlz4_frames_batch_info_dev: max_decoded int64, status uint8 (CUDA tensors, one entry per frame)."""
+    ctx.check(api.lib().dlz4_frames_batch_info_dev(ctx.handle, _p(src), _p(frame_off), _p(frame_len), frame_off.numel(), _p(max_decoded),
+                                                   _p(status), _stream()))
+
+
+def frames_decompress_batch_dev(ctx, src, frame_off, frame_len, dst, dst_off, dst_cap, out_len, status, dictionary=None, flags=1):
+    """dlz4_frames_decompress_batch_dev on the current torch stream; per-frame statuses land in `status` (uint8)."""
+    ctx.check(api.lib().dlz4_frames_decompress_batch_dev(ctx.handle, _p(src), _p(frame_off), _p(frame_len), frame_off.numel(),
+                                                         _p(dictionary), dictionary.numel() if dictionary is not None else 0,
+                                                         int(flags), _p(dst), _p(dst_off), _p(dst_cap), _p(out_len), _p(status),
+                                                         _stream()))

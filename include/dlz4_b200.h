@@ -199,6 +199,47 @@ int dlz4_frame_decompress(dlz4_ctx *ctx, const uint8_t *frame, uint64_t frame_le
                           uint64_t dict_len, uint32_t flags, uint8_t *output, uint64_t output_cap,
                           uint64_t *output_len);
 
+/* ---- batched frames: LZ4.compress / LZ4.decompress once per message, for many messages in one GPU pass ----
+ * Every frame of a batch shares one option set (opts on compress, flags on decompress) and one optional dictionary; frame i
+ * comes out exactly as the single-frame call makes it, byte for byte and status for status.  Per-frame work is one thread or
+ * one warp per frame; inside a frame the block table stays a short serial loop.  This is the path for many small frames: one
+ * warp per frame decodes a batch of a few large frames more slowly than dlz4_frame_decompress's jump decoder, and a linked
+ * frame of several blocks compresses on one warp instead of the segment engine (the crossover is measured by
+ * tools/frame_batch_bench.py and recorded in DESIGN.md).
+ * _dev variants take device pointers, queue their work on `stream` and synchronise it once, to read the block count back.
+ * Host variants stage through the context's scratch (pageable memory works) and return when the results are in place.
+ * A frame of 0x7FFF0000 bytes or more makes the call return DLZ4_E_TOO_LARGE, as dlz4_frame_compress does.
+ *
+ * Compress: frame i = dlz4_frame_compress(src[src_off[i] .. +src_len[i]), dictionary, opts), frames packed back to back:
+ *   frame i is dst[frame_off[i] .. frame_off[i+1]) (frame_off has nframes + 1 entries).  dst_cap must be at least the sum of
+ *   dlz4_frame_bound(src_len[i]) (else DLZ4_E_OUTPUT_TOO_SMALL).  max_len: an upper bound of src_len[] (_dev only).
+ *   Host variant: src holds src_bytes bytes, dst dst_cap bytes. */
+int dlz4_frames_compress_batch_dev(dlz4_ctx *ctx, const uint8_t *src, const uint64_t *src_off, const uint32_t *src_len,
+                                   uint32_t nframes, uint32_t max_len, const uint8_t *dictionary, uint32_t dict_len,
+                                   const dlz4_frame_opts *opts /* host */, uint8_t *dst, uint64_t dst_cap, uint64_t *frame_off,
+                                   void *stream);
+int dlz4_frames_compress_batch(dlz4_ctx *ctx, const uint8_t *src, uint64_t src_bytes, const uint64_t *src_off,
+                               const uint32_t *src_len, uint32_t nframes, const uint8_t *dictionary, uint32_t dict_len,
+                               const dlz4_frame_opts *opts, uint8_t *dst, uint64_t dst_cap, uint64_t *frame_off);
+/* Sizing pass: max_decoded[i] = dlz4_frame_info(frame i).max_decoded, status[i] = its status (0, 2, 5 or 6; max_decoded[i] = 0
+ * on error).  Frame i is src[frame_off[i] .. +frame_len[i]). */
+int dlz4_frames_batch_info_dev(dlz4_ctx *ctx, const uint8_t *src, const uint64_t *frame_off, const uint64_t *frame_len,
+                               uint32_t nframes, uint64_t *max_decoded, uint8_t *status, void *stream);
+int dlz4_frames_batch_info(dlz4_ctx *ctx, const uint8_t *src, uint64_t src_bytes, const uint64_t *frame_off,
+                           const uint64_t *frame_len, uint32_t nframes, uint64_t *max_decoded, uint8_t *status);
+/* Decompress: the first frame in src[frame_off[i] .. +frame_len[i]) (bytes after it are ignored, as in the single-frame call)
+ *   decodes to dst[dst_off[i] .. +dst_cap[i]); status[i] / out_len[i] are what dlz4_frame_decompress(frame i, dictionary, flags,
+ *   output_cap = dst_cap[i]) returns (out_len[i] = 0 on error).  Bytes of dst[dst_off[i] + out_len[i] .. +dst_cap[i]) are
+ *   unspecified afterwards.  The host variant returns the first non-zero status, like dlz4_decompress_blocks. */
+int dlz4_frames_decompress_batch_dev(dlz4_ctx *ctx, const uint8_t *src, const uint64_t *frame_off, const uint64_t *frame_len,
+                                     uint32_t nframes, const uint8_t *dictionary, uint32_t dict_len, uint32_t flags,
+                                     uint8_t *dst, const uint64_t *dst_off, const uint64_t *dst_cap, uint64_t *out_len,
+                                     uint8_t *status, void *stream);
+int dlz4_frames_decompress_batch(dlz4_ctx *ctx, const uint8_t *src, uint64_t src_bytes, const uint64_t *frame_off,
+                                 const uint64_t *frame_len, uint32_t nframes, const uint8_t *dictionary, uint32_t dict_len,
+                                 uint32_t flags, uint8_t *dst, uint64_t dst_bytes, const uint64_t *dst_off,
+                                 const uint64_t *dst_cap, uint64_t *out_len, uint8_t *status);
+
 /* SURVEY 8 f3: a buffer of several concatenated frames (what `cat a.lz4 b.lz4` or the lz4 CLI with several inputs produces) with
  * skippable frames (magic 0x184D2A50..5F, u32 size, payload) between them.  bufferDecompress.js:51-220 stops at the first
  * EndMark; the reference's stream decoder loops over frames (src/shared/lz4Decode.js:262-266).  Decodes every LZ4 frame in
