@@ -13,10 +13,10 @@ def _p(t):
     return C.c_void_p(t.data_ptr()) if t is not None and t.numel() else None
 
 
-def _stream():
-    """Current torch stream as the ABI's opaque handle.  torch's default stream has handle 0, which the ABI reads as
-    "use the context's own stream", so it is passed as cudaStreamLegacy (0x1) instead."""
-    h = torch.cuda.current_stream().cuda_stream
+def _stream(device=None):
+    """Current torch stream (of `device`, default the current device) as the ABI's opaque handle.  torch's default stream has
+    handle 0, which the ABI reads as "use the context's own stream", so it is passed as cudaStreamLegacy (0x1) instead."""
+    h = torch.cuda.current_stream(device).cuda_stream
     return C.c_void_p(h if h else 1)
 
 
@@ -82,3 +82,80 @@ def frames_decompress_batch_dev(ctx, src, frame_off, frame_len, dst, dst_off, ds
                                                          _p(dictionary), dictionary.numel() if dictionary is not None else 0,
                                                          int(flags), _p(dst), _p(dst_off), _p(dst_cap), _p(out_len), _p(status),
                                                          _stream()))
+
+
+# ---------------------------------------------------------------------------------------------- single frames in device memory
+def frame_compress_dev(ctx, src, dst, opts, dictionary=None):
+    """dlz4_frame_compress_dev on the current torch stream.  src/dst/dictionary are uint8 CUDA tensors (any byte offset), dst
+    at least api.frame_bound(src.numel()) bytes; opts an api.FrameOpts (api.frame_opts(...)).  Returns the frame's length."""
+    n = C.c_uint64(0)
+    ctx.check(api.lib().dlz4_frame_compress_dev(ctx.handle, _p(src), src.numel(), _p(dictionary),
+                                                dictionary.numel() if dictionary is not None else 0, C.byref(opts), _p(dst), dst.numel(),
+                                                C.byref(n), _stream(src.device)))
+    return int(n.value)
+
+
+def frame_info_dev(ctx, frame):
+    """dlz4_frame_info_dev on the current torch stream: the api.FrameInfo of the frame in a uint8 CUDA tensor.  Raises
+    api.LZ4Error with the reference's text, as api.frame_info does."""
+    info = api.FrameInfo()
+    st = api.lib().dlz4_frame_info_dev(ctx.handle, _p(frame), frame.numel(), C.byref(info), _stream(frame.device))
+    ctx.check(st, " %d" % info.version if st == api.E_BAD_VERSION else "")
+    return info
+
+
+def frame_decompress_dev(ctx, frame, dst, dictionary=None, flags=1):
+    """dlz4_frame_decompress_dev on the current torch stream: decodes the frame in `frame` into `dst` (uint8 CUDA tensors, the
+    capacity is dst.numel()).  flags: bit 0 content checksum, bit 1 block checksums, bit 2 header checksum.  Returns the
+    decoded length."""
+    n = C.c_uint64(0)
+    ctx.check(api.lib().dlz4_frame_decompress_dev(ctx.handle, _p(frame), frame.numel(), _p(dictionary),
+                                                  dictionary.numel() if dictionary is not None else 0, int(flags), _p(dst), dst.numel(),
+                                                  C.byref(n), _stream(frame.device)))
+    return int(n.value)
+
+
+def _bytes_of(t, name, ctx):
+    """A contiguous CUDA tensor viewed as uint8 bytes, on the context's device."""
+    if not isinstance(t, torch.Tensor) or not t.is_cuda:
+        raise ValueError("%s must be a CUDA tensor" % name)
+    if not t.is_contiguous():
+        raise ValueError("%s must be contiguous" % name)
+    if ctx is not None and t.device.index != ctx.device:
+        raise ValueError("%s is on %s, the context on cuda:%d" % (name, t.device, ctx.device))
+    return t.reshape(-1).view(torch.uint8)
+
+
+def _dictionary_on(dictionary, device, ctx):
+    if dictionary is None:
+        return None
+    if isinstance(dictionary, torch.Tensor):
+        d = _bytes_of(dictionary, "dictionary", ctx)
+    else:
+        d = torch.from_numpy(api.ensureBuffer(dictionary).copy()).to(device)
+    return d if d.numel() else None
+
+
+def compress_tensor(t, dictionary=None, maxBlockSize=4194304, blockIndependence=False, contentChecksum=False, addContentSize=True,
+                    blockChecksum=False, ctx=None):
+    """LZ4.compress of a CUDA tensor's bytes, on the GPU end to end: returns a uint8 CUDA tensor of exactly the frame's length,
+    byte-identical to compressBuffer(t's bytes, ...).  t: any contiguous CUDA tensor; dictionary: a CUDA tensor or bytes-like.
+    Runs on the current torch stream and returns when the frame is complete."""
+    src = _bytes_of(t, "t", ctx)
+    ctx = ctx or api.default_context(src.device.index)
+    d = _dictionary_on(dictionary, src.device, ctx)
+    dst = torch.empty(api.frame_bound(src.numel()), dtype=torch.uint8, device=src.device)
+    n = frame_compress_dev(ctx, src, dst, api.frame_opts(maxBlockSize, blockIndependence, contentChecksum, addContentSize, blockChecksum), d)
+    return dst[:n]
+
+
+def decompress_tensor(frame, dictionary=None, verifyChecksum=True, verifyBlockChecksums=False, ctx=None):
+    """LZ4.decompress of a frame held in a CUDA tensor, on the GPU end to end: returns the decoded bytes as a uint8 CUDA tensor
+    (sized with frame_info_dev).  Raises api.LZ4Error with the reference's text, as decompressBuffer does."""
+    f = _bytes_of(frame, "frame", ctx)
+    ctx = ctx or api.default_context(f.device.index)
+    d = _dictionary_on(dictionary, f.device, ctx)
+    info = frame_info_dev(ctx, f)
+    out = torch.empty(int(info.max_decoded), dtype=torch.uint8, device=f.device)
+    n = frame_decompress_dev(ctx, f, out, d, (1 if verifyChecksum else 0) | (2 if verifyBlockChecksums else 0))
+    return out[:n]

@@ -199,6 +199,33 @@ int dlz4_frame_decompress(dlz4_ctx *ctx, const uint8_t *frame, uint64_t frame_le
                           uint64_t dict_len, uint32_t flags, uint8_t *output, uint64_t output_cap,
                           uint64_t *output_len);
 
+/* ---- single frames in device memory: dlz4_frame_compress / dlz4_frame_info / dlz4_frame_decompress on CUDA buffers ----
+ * src, dictionary, frame and dst are device pointers of any alignment; every other pointer is host memory.  A call stages
+ * what it reads in the context's scratch with one device-to-device copy, then runs the host call's code paths (the
+ * segment-parallel compressor, the jump decoder, ...) and produces the same bytes and statuses.  Work is queued on `stream`
+ * (NULL = the context's stream), and the call has synchronised `stream` when it returns, because its results are host values:
+ *   compress:   twice -- once for the compressed body's length (it places the EndMark and sizes *frame_len), once at the end.
+ *   info:       once -- for the header bytes and the block walk's count, bound and end.
+ *   decompress: three times (twice for a frame without blocks, or on an error found before decoding) plus the decode
+ *               route's own one or two -- for the header and the block count, for the block table
+ *               (it sizes the jump decoder's scratch and selects the decode route), and for the final status.
+ * Not covered: concatenated / skippable frames and block ranges (use the host calls), and the stream classes. */
+/* dlz4_frame_compress on device memory.  dst_cap must be at least dlz4_frame_bound(src_len) (else DLZ4_E_OUTPUT_TOO_SMALL;
+ * no silent truncation here).  *frame_len (host) = the frame's length.  The independent 64 KiB-block frames that the host call
+ * sends through its chunked PCIe pipeline take the ordinary block compressor here; the bytes are the same. */
+int dlz4_frame_compress_dev(dlz4_ctx *ctx, const uint8_t *src, uint64_t src_len, const uint8_t *dictionary, uint64_t dict_len,
+                            const dlz4_frame_opts *opts /* host */, uint8_t *dst, uint64_t dst_cap, uint64_t *frame_len,
+                            void *stream);
+/* dlz4_frame_info on a frame in device memory: same fields, same status for every input. */
+int dlz4_frame_info_dev(dlz4_ctx *ctx, const uint8_t *frame, uint64_t frame_len, dlz4_frame_info_t *info /* host */,
+                        void *stream);
+/* dlz4_frame_decompress on device memory: same flags.  Return value and *output_len (host) are what dlz4_frame_decompress
+ * returns for the same bytes, dictionary, flags and output_cap.  dst bytes beyond *output_len, and all of dst on error, are
+ * unspecified.  Checksums are computed and compared on the device. */
+int dlz4_frame_decompress_dev(dlz4_ctx *ctx, const uint8_t *frame, uint64_t frame_len, const uint8_t *dictionary,
+                              uint64_t dict_len, uint32_t flags, uint8_t *dst, uint64_t output_cap, uint64_t *output_len,
+                              void *stream);
+
 /* ---- batched frames: LZ4.compress / LZ4.decompress once per message, for many messages in one GPU pass ----
  * Every frame of a batch shares one option set (opts on compress, flags on decompress) and one optional dictionary; frame i
  * comes out exactly as the single-frame call makes it, byte for byte and status for status.  Per-frame work is one thread or
