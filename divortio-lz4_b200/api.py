@@ -133,6 +133,10 @@ def lib():
         "dlz4_frame_compress_dev": (C.c_int, [vp, vp, u64, vp, u64, C.POINTER(FrameOpts), vp, u64, C.POINTER(u64), vp]),
         "dlz4_frame_info_dev": (C.c_int, [vp, vp, u64, C.POINTER(FrameInfo), vp]),
         "dlz4_frame_decompress_dev": (C.c_int, [vp, vp, u64, vp, u64, u32, vp, u64, C.POINTER(u64), vp]),
+        "dlz4_frames_compress_dev": (C.c_int, [vp, vp, u64, u64, vp, u64, C.POINTER(FrameOpts), vp, u64, vp, C.POINTER(u64),
+                                               C.POINTER(u32), vp]),
+        "dlz4_frames_info_dev": (C.c_int, [vp, vp, u64, C.POINTER(u64), C.POINTER(u32), vp]),
+        "dlz4_frames_decompress_dev": (C.c_int, [vp, vp, u64, vp, u64, u32, vp, u64, C.POINTER(u64), C.POINTER(u32), vp]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(L, name)
@@ -151,7 +155,7 @@ EXPORTED_SYMBOLS = [
     "dlz4_chain_compress", "dlz4_stream_blocks", "dlz4_frame_body_compress", "dlz4_frame_body_fetch", "dlz4_frame_header", "dlz4_frame_decompress_range",
     "dlz4_xxh32_update_resident", "dlz4_frames_compress_batch_dev", "dlz4_frames_compress_batch", "dlz4_frames_batch_info_dev",
     "dlz4_frames_batch_info", "dlz4_frames_decompress_batch_dev", "dlz4_frames_decompress_batch", "dlz4_frame_compress_dev",
-    "dlz4_frame_info_dev", "dlz4_frame_decompress_dev",
+    "dlz4_frame_info_dev", "dlz4_frame_decompress_dev", "dlz4_frames_compress_dev", "dlz4_frames_info_dev", "dlz4_frames_decompress_dev",
 ]
 
 

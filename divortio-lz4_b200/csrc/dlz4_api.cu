@@ -43,5 +43,6 @@ extern "C" {
 #include "api_frame_decompress.inc"
 #include "api_frame_batch.inc"
 #include "api_frame_dev.inc"
+#include "api_frames_dev.inc"
 #include "api_stream.inc"
 }  // extern "C"

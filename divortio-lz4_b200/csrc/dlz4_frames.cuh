@@ -416,4 +416,88 @@ __global__ void __launch_bounds__(256) k_fd_finish(const uint8_t *__restrict__ s
     out_len[f] = st ? 0 : total[f];
 }
 
+// ------------------------------------------------------------------ frame sequences (dlz4_frames_*_dev, api_frames_dev.inc)
+struct FsWalk {                                                  // what k_fs_walk found
+    unsigned long long count, max_decoded;                       // LZ4 frames before the first error, sum of their max_decoded
+    uint32_t status, pad;                                        // for_each_frame's status
+};
+
+// One thread: for_each_frame over data[0, len) (skippable frames skipped) with dlz4_frame_info per LZ4 frame, in the host
+// order; stops at the first error.  Frame k (k < cap) gets its offset, frame_bytes and max_decoded; `count` is the true number
+// of frames, so a caller whose arrays were too small can grow them and run the walk again.  Reads bytewise: any alignment,
+// nothing behind data + len.
+__global__ void __launch_bounds__(32) k_fs_walk(const uint8_t *__restrict__ data, uint64_t len, uint32_t cap, uint64_t *frame_off,
+                                                uint64_t *frame_len, uint64_t *max_decoded, FsWalk *res) {
+    if (threadIdx.x != 0) return;
+    uint64_t pos = 0, count = 0, sum = 0;
+    uint32_t st = 0;
+    while (pos < len) {
+        if (pos + 4 > len) { st = 5; break; }
+        if ((ld32b(data + pos) & 0xFFFFFFF0u) == 0x184D2A50u) {  // skippable frame: magic, u32 size, payload
+            if (pos + 8 > len) { st = 2; break; }
+            const uint64_t sz = ld32b(data + pos + 4);
+            if (pos + 8 + sz > len) { st = 2; break; }
+            pos += 8 + sz;
+            continue;
+        }
+        const uint8_t *p = data + pos;                           // dlz4_frame_info(p, L): parse_header, walk_blocks, frame_bytes
+        const uint64_t L = len - pos;
+        if (ld32b(p) != 0x184D2204u) { st = 5; break; }
+        if (L < 5) { st = 6; break; }
+        uint64_t q = 4, content = 0, bound = 0;
+        const uint8_t flg = p[q++];
+        if (((flg & 0xC0) >> 6) != 1) { st = 6; break; }
+        if (q >= L) { st = 2; break; }
+        const uint32_t bid = (p[q++] >> 4) & 7;
+        const uint32_t bmax = bid >= 4 ? (65536u << (2 * (bid - 4))) : 4194304u;
+        if (flg & 0x08) {
+            if (q + 8 > L) { st = 2; break; }
+            content = (uint64_t)ld32b(p + q) | ((uint64_t)ld32b(p + q + 4) << 32);
+            q += 8;
+        }
+        if (flg & 0x01) { if (q + 4 > L) { st = 2; break; } q += 4; }
+        q += 1;
+        if (q > L) { st = 2; break; }
+        while (q < L) {
+            if (q + 4 > L) { st = 2; break; }
+            const uint32_t bs = ld32b(p + q);
+            q += 4;
+            if (bs == 0) break;
+            const uint32_t actual = bs & 0x7FFFFFFFu;
+            if (q + actual > L) { st = 2; break; }
+            bound += (bs >> 31) ? actual : ((uint64_t)actual * 255 < bmax ? (uint64_t)actual * 255 : bmax);
+            q += actual;
+            if (flg & 0x10) { if (q + 4 > L) { st = 2; break; } q += 4; }
+        }
+        if (st) break;
+        const uint64_t fb = q + ((flg & 0x04) ? 4 : 0);
+        if (fb > L) { st = 2; break; }
+        const uint64_t md = content ? content : bound;
+        if (count < cap) { frame_off[count] = pos; frame_len[count] = fb; max_decoded[count] = md; }
+        ++count;
+        sum += md;
+        pos += fb;
+    }
+    res->count = count;
+    res->max_decoded = sum;
+    res->status = st;
+    res->pad = 0;
+}
+
+// One warp per frame: the out_len[f] bytes decoded into scratch at soff[f] move to dst at doff[f] (a group of small frames
+// decoded at a scan of their max_decoded, gathered to their running offsets).
+__global__ void __launch_bounds__(256) k_fs_gather(const uint8_t *__restrict__ scratch, const uint64_t *__restrict__ soff,
+                                                   const uint64_t *__restrict__ out_len, const uint64_t *__restrict__ doff, uint32_t n,
+                                                   uint8_t *dst) {
+    const uint32_t lane = lane_id();
+    for (uint32_t f = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; f < n; f += (gridDim.x * blockDim.x) >> 5) {
+        const uint8_t *s = scratch + soff[f];
+        uint8_t *d = dst + doff[f];
+        const uint64_t len = out_len[f];
+        for (uint64_t o = 0; o < len; o += 1u << 20)
+            warp_copy(d + o, s + o, (uint32_t)(len - o < (1u << 20) ? len - o : (1u << 20)), lane);
+        __syncwarp();
+    }
+}
+
 }  // namespace dlz4

@@ -6,7 +6,7 @@ import ctypes as C
 
 import torch
 
-from . import api
+from . import api, sharded
 
 
 def _p(t):
@@ -159,3 +159,63 @@ def decompress_tensor(frame, dictionary=None, verifyChecksum=True, verifyBlockCh
     out = torch.empty(int(info.max_decoded), dtype=torch.uint8, device=f.device)
     n = frame_decompress_dev(ctx, f, out, d, (1 if verifyChecksum else 0) | (2 if verifyBlockChecksums else 0))
     return out[:n]
+
+
+# ---------------------------------------------------------------------------------------- concatenated frames in device memory
+def frames_compress_dev(ctx, src, frame_bytes, dst, opts, dictionary=None):
+    """dlz4_frames_compress_dev on the current torch stream: src cut into spans of frame_bytes, one frame each, back to back in
+    dst (uint8 CUDA tensors, dst at least the sum of api.frame_bound over the spans).  Returns (length, frame_off list)."""
+    n, k = C.c_uint64(0), C.c_uint32(0)
+    spans = max(1, -(-src.numel() // int(frame_bytes))) if frame_bytes else 1
+    off = (C.c_uint64 * (spans + 1))()
+    ctx.check(api.lib().dlz4_frames_compress_dev(ctx.handle, _p(src), src.numel(), int(frame_bytes), _p(dictionary),
+                                                 dictionary.numel() if dictionary is not None else 0, C.byref(opts), _p(dst),
+                                                 dst.numel(), off, C.byref(n), C.byref(k), _stream(src.device)))
+    return int(n.value), [int(x) for x in off[:k.value + 1]]
+
+
+def frames_info_dev(ctx, data):
+    """dlz4_frames_info_dev on the current torch stream: (sum of max_decoded, LZ4 frames) of the concatenated frames in a uint8
+    CUDA tensor.  Raises api.LZ4Error as api.decompressFrames does."""
+    total, count = C.c_uint64(0), C.c_uint32(0)
+    ctx.check(api.lib().dlz4_frames_info_dev(ctx.handle, _p(data), data.numel(), C.byref(total), C.byref(count), _stream(data.device)))
+    return int(total.value), int(count.value)
+
+
+def frames_decompress_dev(ctx, data, dst, dictionary=None, flags=1):
+    """dlz4_frames_decompress_dev on the current torch stream: every LZ4 frame of `data` in order into `dst` (capacity
+    dst.numel()), skippable frames skipped.  Returns (decoded length, frames)."""
+    n, count = C.c_uint64(0), C.c_uint32(0)
+    ctx.check(api.lib().dlz4_frames_decompress_dev(ctx.handle, _p(data), data.numel(), _p(dictionary),
+                                                   dictionary.numel() if dictionary is not None else 0, int(flags), _p(dst), dst.numel(),
+                                                   C.byref(n), C.byref(count), _stream(data.device)))
+    return int(n.value), int(count.value)
+
+
+def compress_tensor_frames(t, dictionary=None, maxBlockSize=4194304, blockIndependence=False, contentChecksum=False,
+                           addContentSize=True, blockChecksum=False, frame_max=sharded.FRAME_MAX, ctx=None):
+    """compress_tensor for a CUDA tensor of any size: frames cut by sharded.frame_spans (one frame up to frame_max bytes, else
+    frames of sharded.FRAME_SPLIT bytes, or of frame_max bytes when the caller sets a limit), back to back in one uint8 CUDA
+    tensor.  Up to frame_max bytes the result is compress_tensor's frame; the content checksums of several frames are computed
+    side by side."""
+    src = _bytes_of(t, "t", ctx)
+    ctx = ctx or api.default_context(src.device.index)
+    d = _dictionary_on(dictionary, src.device, ctx)
+    spans = sharded.frame_spans(src.numel(), frame_max)
+    step = max(1, spans[0][1] - spans[0][0])
+    dst = torch.empty(sum(api.frame_bound(hi - lo) for lo, hi in spans), dtype=torch.uint8, device=src.device)
+    n, _ = frames_compress_dev(ctx, src, step, dst,
+                               api.frame_opts(maxBlockSize, blockIndependence, contentChecksum, addContentSize, blockChecksum), d)
+    return dst[:n]
+
+
+def decompress_tensor_frames(data, dictionary=None, verifyChecksum=True, verifyBlockChecksums=False, ctx=None):
+    """api.decompressFrames of concatenated frames held in a CUDA tensor, on the GPU end to end: returns (uint8 CUDA tensor of
+    the decoded bytes, number of LZ4 frames).  Raises api.LZ4Error with the reference's text."""
+    f = _bytes_of(data, "data", ctx)
+    ctx = ctx or api.default_context(f.device.index)
+    d = _dictionary_on(dictionary, f.device, ctx)
+    total, _ = frames_info_dev(ctx, f)
+    out = torch.empty(total, dtype=torch.uint8, device=f.device)
+    n, count = frames_decompress_dev(ctx, f, out, d, (1 if verifyChecksum else 0) | (2 if verifyBlockChecksums else 0))
+    return out[:n], count

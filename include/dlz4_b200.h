@@ -209,7 +209,8 @@ int dlz4_frame_decompress(dlz4_ctx *ctx, const uint8_t *frame, uint64_t frame_le
  *   decompress: three times (twice for a frame without blocks, or on an error found before decoding) plus the decode
  *               route's own one or two -- for the header and the block count, for the block table
  *               (it sizes the jump decoder's scratch and selects the decode route), and for the final status.
- * Not covered: concatenated / skippable frames and block ranges (use the host calls), and the stream classes. */
+ * Not covered: block ranges (use the host calls) and the stream classes.  Concatenated and skippable frames: the
+ * dlz4_frames_*_dev calls below. */
 /* dlz4_frame_compress on device memory.  dst_cap must be at least dlz4_frame_bound(src_len) (else DLZ4_E_OUTPUT_TOO_SMALL;
  * no silent truncation here).  *frame_len (host) = the frame's length.  The independent 64 KiB-block frames that the host call
  * sends through its chunked PCIe pipeline take the ordinary block compressor here; the bytes are the same. */
@@ -277,6 +278,32 @@ int dlz4_frames_decompress(dlz4_ctx *ctx, const uint8_t *data, uint64_t data_len
                            uint32_t flags, uint8_t *output, uint64_t output_cap, uint64_t *output_len, uint32_t *frames);
 /* Sum of the decoded-size bounds of all LZ4 frames in `data` (to size `output`), and their count. */
 int dlz4_frames_info(const uint8_t *data, uint64_t data_len, uint64_t *max_decoded, uint32_t *frames);
+
+/* ---- concatenated frames in device memory: inputs of any size, and the frame loop above, on CUDA buffers ----
+ * Pointer conventions of dlz4_frame_*_dev: src, dictionary, data and dst are device pointers of any alignment and without
+ * slack after their end; every other pointer is host memory; work is queued on `stream` (NULL = the context's stream).
+ *
+ * Compress: frame k = dlz4_frame_compress(src[k*frame_bytes .. min((k+1)*frame_bytes, src_len)), dictionary, opts), frames back
+ *   to back in dst (src_len == 0 gives one empty frame).  1 <= frame_bytes < 0x7FFF0000 (else DLZ4_E_INVALID_ARG /
+ *   DLZ4_E_TOO_LARGE).  dst_cap must be at least the sum of dlz4_frame_bound over the spans (else DLZ4_E_OUTPUT_TOO_SMALL, before
+ *   any work).  frame_off (nullable) receives nframes + 1 entries: frame k is dst[frame_off[k] .. frame_off[k+1]).  The content
+ *   checksums of all frames run side by side, one serial chain each, beside the block work.  `stream` is synchronised once per
+ *   frame (its body length places the next frame) and once at the end.
+ * Info: dlz4_frames_info on device memory -- the same *max_decoded, *frames and status for every input.  One synchronisation.
+ * Decompress: dlz4_frames_decompress on device memory -- the same return value, *output_len and *frames as the host call for
+ *   the same bytes, dictionary, flags and output_cap.  dst beyond *output_len, and all of dst on error, are unspecified.
+ *   Frames whose max_decoded is below a size threshold decode in groups, one warp per frame; larger ones one at a time
+ *   through dlz4_frame_decompress_dev's decoders.  `stream` is synchronised for the frame walk (twice when the sequence has
+ *   more than 4096 frames), for the parse, once per group of small frames, for each large frame's block table and decode
+ *   route, and once at the end for the statuses. */
+int dlz4_frames_compress_dev(dlz4_ctx *ctx, const uint8_t *src, uint64_t src_len, uint64_t frame_bytes, const uint8_t *dictionary,
+                             uint64_t dict_len, const dlz4_frame_opts *opts /* host */, uint8_t *dst, uint64_t dst_cap,
+                             uint64_t *frame_off, uint64_t *out_len, uint32_t *nframes, void *stream);
+int dlz4_frames_info_dev(dlz4_ctx *ctx, const uint8_t *data, uint64_t data_len, uint64_t *max_decoded, uint32_t *frames,
+                         void *stream);
+int dlz4_frames_decompress_dev(dlz4_ctx *ctx, const uint8_t *data, uint64_t data_len, const uint8_t *dictionary,
+                               uint64_t dict_len, uint32_t flags, uint8_t *dst, uint64_t output_cap, uint64_t *output_len,
+                               uint32_t *frames, void *stream);
 
 /* SURVEY 8 f1 (streaming codec, src/shared/lz4Encode.js / lz4Decode.js) -- the two pieces the stream classes need below them.
  *
