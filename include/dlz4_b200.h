@@ -106,6 +106,9 @@ void dlz4_shard_range(uint64_t nblocks, uint32_t world, uint32_t rank, uint64_t 
  *   max_block_len: an upper bound of src_len[] known to the caller (0xFFFFFFFF if unknown); blocks of at most
  *   64 KiB with no prefix and DLZ4_WARM_NONE take the match finder + encoder pair (k_parse_pw, k_encode_blocks); batches of
  *   uniform blocks > 64 KiB are cut into segments (the call then reads the descriptors back and synchronises the stream).
+ *   The match finder's record scratch is (max_block_len / 4 + 2) x 8 bytes per block, kept by the context and capped at
+ *   2.25 GiB per launch: a larger batch (more than 16 384 blocks of 64 KiB, or many small blocks behind one 64 KiB block)
+ *   runs as several launches on `stream`.  Growing the scratch synchronises the device.
  */
 int dlz4_compress_blocks_dev(dlz4_ctx *ctx, const uint8_t *src, const uint64_t *src_off, const uint32_t *src_len,
                              uint32_t nblocks, uint32_t max_block_len, const uint8_t *prefix, uint32_t prefix_len, int warm,
